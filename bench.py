@@ -2,6 +2,7 @@
 """bench.py — images/sec of the PASSL self-supervised hot path on B200 (BASELINE.json metric).
 
   python bench.py --gpus N --steps K --warmup W [--config c2|c3|c4|c5]     (N>1: launched by torch.distributed.run, one rank per GPU)
+  python bench.py ... --dump-outputs DIR                                   also writes what the last timed step computed (seeded inputs)
   python bench.py --impl reference ...                                     the reference math on the host CPU cores (oracle port)
 
 Workloads (BASELINE.json `configs`; default c2 = the one the metric is quoted on):
@@ -376,6 +377,27 @@ def bench_infonce(dev, pk):
                       % (NQ, NQ, NQ * D * Kq * 2 >> 20, NQ)}
 
 
+DUMP_SAMPLE = 4 << 20          # elements kept of each dumped buffer: params + grads stay at 32 MB for every config
+
+
+def dump_outputs(path, loss, store):
+    """What the last timed step hands back, as float32 .npy files: `loss`, and the parameters it updated (`params`, the fp32
+    master buffer of the ParamStore) with the gradients it updated them from (`grads`).  Buffers longer than DUMP_SAMPLE are
+    sampled at positions drawn from a fixed seed.  The step itself sums split-K partials in a fixed order, so two runs with the
+    same arguments write the same bits (c2, measured on a B200 at 1000 W)."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    idx = None
+    if store.numel > DUMP_SAMPLE:
+        pick = np.sort(np.random.default_rng(0).choice(store.numel, size=DUMP_SAMPLE, replace=False))
+        idx = torch.from_numpy(pick).to(store.master.device)
+    for name, t in (("loss", loss.detach().reshape(())), ("params", store.master), ("grads", store.grad)):
+        if t.dim() and idx is not None:
+            t = t[idx]
+        np.save(os.path.join(path, name + ".npy"), t.float().cpu().numpy())
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -438,6 +460,8 @@ def run_ours(args):
     sampler.stop_flag = True
     loss_val = float(loss.item())
     value = B * world * args.steps / (ms / 1e3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, loss, wl["store"])
 
     # ---- e2e: inputs from pinned host memory every step + D2H read of the loss -------------------------------------
     # The user-facing loop (engine/trainer.py IterLoader with prefetch) double-buffers the input: the H2D copy of step t+1 runs
@@ -605,7 +629,13 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default="c2", choices=["c2", "c3", "c4", "c5"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the loss, parameters and gradients of the last timed step "
+                                                          "to DIR/<name>.npy (float32, sampled to <= 32 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     # The contract is ONE JSON line on stdout.  Libraries write there too (NCCL prints "NCCL version ..." from its C side at
     # communicator creation): everything goes to stderr while the run is in progress, the real stdout comes back for the result line.
     sys.stdout.flush()

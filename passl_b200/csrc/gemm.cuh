@@ -70,6 +70,8 @@ struct GemmParams {
   long long ldc;        // elements between consecutive output rows (pixels)
   int out_fp32;         // 0: bf16, 1: fp32
   int atomic_add;       // fp32 only: red.add instead of store (split-K / wgrad)
+  float* partial;       // atomic_add with splits > 1: split s stores its tile to partial + s * part_stride (same
+  long long part_stride; // addressing as out); splitk_reduce adds the slices into out in split order
   int out_pixel;        // 1: row -> NHWC pixel address through geom + (OH, OW, osh, osw, oh0, ow0)
   int OH, OW, osh, osw, oh0, ow0;
   const float* bias;            // [N] or null
@@ -1048,7 +1050,13 @@ __global__ void __launch_bounds__(64 + 32 * EW, 1) gemm_tcgen05_kernel(const __g
           }
           if (row_ok) {
             float* op = reinterpret_cast<float*>(p.out) + row_off + oc0;
-            if (p.atomic_add) {
+            if (p.partial) {
+              float* pp = p.partial + (size_t)(tile % p.splits) * p.part_stride + row_off + oc0;
+#pragma unroll
+              for (int j4 = 0; j4 < 8; ++j4)      // ldc % 4 == 0 (splitk path precondition): 16-byte aligned like out
+                if (cc0 + j4 * 4 < col_lim)
+                  *reinterpret_cast<float4*>(pp + j4 * 4) = make_float4(f[j4 * 4], f[j4 * 4 + 1], f[j4 * 4 + 2], f[j4 * 4 + 3]);
+            } else if (p.atomic_add) {
 #pragma unroll
               for (int j = 0; j < 32; ++j)
                 if (cc0 + j < col_lim) red_add_f32(op + j, f[j]);

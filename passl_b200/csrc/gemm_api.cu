@@ -6,6 +6,8 @@
 
 #include <string.h>
 
+#include <mutex>
+
 namespace pb {
 
 // 128 x 128 bf16 identity used as the A operand of the residual-through-the-tensor-pipe iterations (gemm.cuh, res_iters)
@@ -108,8 +110,87 @@ static bool pair_eligible(const GemmParams& p, int BN, int BK, bool a_mn) {
          p.k_iters >= mink && (long long)((p.m_blocks + 1) / 2) * p.n_blocks * p.splits >= num_sms() / 2;
 }
 
+// Split-K partial sums are added in a fixed order so that a launch computes the same bits every run (float red.add in
+// whatever order the CTAs finish does not).  The slices live in stream-ordered scratch from a memory pool of this library's own
+// per device, which keeps what it has allocated (its peak is one step's largest concurrent slices) instead of returning it to
+// the driver at every synchronisation; the device's default pool and the framework's allocator are left alone.
+int splitk_scratch(float** out, size_t n_floats, cudaStream_t st) {
+  constexpr int kMaxDevices = 64;
+  static cudaMemPool_t pools[kMaxDevices] = {};
+  static std::mutex mu;
+  int dev = 0;
+  PB_CUDA_CHECK(cudaGetDevice(&dev));
+  if (dev < 0 || dev >= kMaxDevices) return PB_ERR_UNSUPPORTED;
+  cudaMemPool_t pool;
+  {
+    std::lock_guard<std::mutex> lock(mu);
+    if (!pools[dev]) {
+      cudaMemPoolProps props;
+      memset(&props, 0, sizeof(props));
+      props.allocType = cudaMemAllocationTypePinned;
+      props.location.type = cudaMemLocationTypeDevice;
+      props.location.id = dev;
+      cudaMemPool_t created;
+      PB_CUDA_CHECK(cudaMemPoolCreate(&created, &props));
+      uint64_t keep = ~0ull;
+      PB_CUDA_CHECK(cudaMemPoolSetAttribute(created, cudaMemPoolAttrReleaseThreshold, &keep));
+      pools[dev] = created;
+    }
+    pool = pools[dev];
+  }
+  PB_CUDA_CHECK(cudaMallocFromPoolAsync(reinterpret_cast<void**>(out), n_floats * sizeof(float), pool, st));
+  return PB_OK;
+}
+
+int splitk_release(float* ptr, cudaStream_t st) {
+  PB_CUDA_CHECK(cudaFreeAsync(ptr, st));
+  return PB_OK;
+}
+
+// out[r * ld + c] += part[0][...] + part[1][...] + ... (slices `stride` floats apart), summed in split order; four columns per
+// thread (cols, ld and stride are multiples of 4)
+__global__ void splitk_reduce_kernel(float* __restrict__ out, const float* __restrict__ part, unsigned rows, unsigned cols4,
+                                     long long ld, long long stride, int splits) {
+  const unsigned n = rows * cols4;
+  for (unsigned e = blockIdx.x * blockDim.x + threadIdx.x; e < n; e += gridDim.x * blockDim.x) {
+    const unsigned r = e / cols4;
+    const long long off = (long long)r * ld + 4ll * (e - r * cols4);
+    float4 s = __ldcs(reinterpret_cast<const float4*>(part + off));
+    for (int k = 1; k < splits; ++k) {
+      const float4 v = __ldcs(reinterpret_cast<const float4*>(part + k * stride + off));
+      s.x += v.x; s.y += v.y; s.z += v.z; s.w += v.w;
+    }
+    float4* o = reinterpret_cast<float4*>(out + off);
+    float4 a = *o;
+    a.x += s.x; a.y += s.y; a.z += s.z; a.w += s.w;
+    *o = a;
+  }
+}
+
+int splitk_reduce(float* out, const float* part, long long rows, long long cols, long long ld, long long stride, int splits,
+                  cudaStream_t st) {
+  if (cols % 4 || ld % 4 || stride % 4 || rows * cols >= (1ll << 32)) return PB_ERR_UNSUPPORTED;
+  const long long n = rows * cols / 4;
+  const long long cap = (long long)num_sms() * 8;
+  const int grid = (int)((n + 255) / 256 < cap ? (n + 255) / 256 : cap);
+  splitk_reduce_kernel<<<grid, 256, 0, st>>>(out, part, (unsigned)rows, (unsigned)(cols / 4), ld, stride, splits);
+  PB_LAUNCH_CHECK();
+  return PB_OK;
+}
+
 static int launch_gemm(const GemmParams& p, int BN, int BK, bool a_mn, bool b_mn, cudaStream_t st, int epi = 0, int cg = 1,
                        bool halo = false, int ew = 8) {
+  if (p.atomic_add && p.splits > 1 && !p.partial) {
+    if (p.ldc % 4 || p.N % 4) return PB_ERR_UNSUPPORTED;
+    GemmParams q = p;
+    q.part_stride = (long long)p.M * p.ldc;
+    int rc = splitk_scratch(&q.partial, (size_t)p.splits * q.part_stride, st);
+    if (rc) return rc;
+    rc = launch_gemm(q, BN, BK, a_mn, b_mn, st, epi, cg, halo, ew);
+    if (!rc) rc = splitk_reduce(reinterpret_cast<float*>(p.out), q.partial, p.M, p.N, p.ldc, q.part_stride, p.splits, st);
+    int rc2 = splitk_release(q.partial, st);
+    return rc ? rc : rc2;
+  }
   if (ew == 16 && epi == 2 && cg == 1 && BN == 256 && BK == 64 && !a_mn && !b_mn && !halo)   // K-small 1x1 convolutions with statistics
     return launch_gemm_t<256, 64, false, false, 2, 1, false, 16>(p, st);
   if (ew == 16 && epi == 1 && BN == 256 && BK == 64 && !a_mn && !halo) {   // epilogue-bound linear launches (GELU / gates)

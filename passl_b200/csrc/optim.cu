@@ -14,6 +14,9 @@
 
 namespace pb {
 
+int splitk_scratch(float** out, size_t n_floats, cudaStream_t st);     // gemm_api.cu: stream-ordered scratch
+int splitk_release(float* ptr, cudaStream_t st);
+
 constexpr int OPT_BLOCK = 1024;  // elements per CTA (256 threads x 4)
 
 __device__ __forceinline__ void store_bf16x4(__nv_bfloat16* dst, const float4& v) {
@@ -42,9 +45,9 @@ __global__ void sgd_momentum_kernel(float* __restrict__ p, const float* __restri
   if (p_bf16) store_bf16x4(p_bf16 + i, pp);
 }
 
-// per-tensor squared norms: norms[2*seg] += sum p^2, norms[2*seg+1] += sum (g*gscale)^2
-__global__ void seg_sqnorm_kernel(const float* __restrict__ p, const float* __restrict__ g, const int* __restrict__ block_seg,
-                                  float* __restrict__ norms, float gscale, long long n) {
+// per-block squared norms: part[2*block] = sum p^2, part[2*block+1] = sum (g*gscale)^2 (seg_norm_finalize_kernel adds them per tensor)
+__global__ void seg_sqnorm_kernel(const float* __restrict__ p, const float* __restrict__ g, float* __restrict__ part, float gscale,
+                                  long long n) {
   __shared__ float red[2][8];
   long long i = ((long long)blockIdx.x * blockDim.x + threadIdx.x) * 4;
   float a = 0.f, b = 0.f;
@@ -62,10 +65,34 @@ __global__ void seg_sqnorm_kernel(const float* __restrict__ p, const float* __re
     a = l < 8 ? red[0][l] : 0.f; b = l < 8 ? red[1][l] : 0.f;
     a = warp_sum(a); b = warp_sum(b);
     if (l == 0) {
-      int s = block_seg[blockIdx.x];
-      red_add_f32(norms + 2 * s, a);
-      red_add_f32(norms + 2 * s + 1, b);
+      part[2 * blockIdx.x] = a;
+      part[2 * blockIdx.x + 1] = b;
     }
+  }
+}
+
+// one CTA per tensor: norms[2*seg + {0,1}] = the sums of that tensor's block partials in a fixed order, so the LARS trust ratio
+// is the same every run (block_seg is non-decreasing: a tensor's blocks are contiguous)
+__global__ void seg_norm_finalize_kernel(const float* __restrict__ part, const int* __restrict__ block_seg, int nblocks,
+                                         float* __restrict__ norms) {
+  __shared__ float red[2][8];
+  const int s = blockIdx.x;
+  int lo = 0, hi = nblocks;
+  while (lo < hi) { const int mid = (lo + hi) >> 1; if (block_seg[mid] < s) lo = mid + 1; else hi = mid; }
+  const int b0 = lo;
+  hi = nblocks;
+  while (lo < hi) { const int mid = (lo + hi) >> 1; if (block_seg[mid] <= s) lo = mid + 1; else hi = mid; }
+  float a = 0.f, b = 0.f;
+  for (int k = b0 + (int)threadIdx.x; k < lo; k += blockDim.x) { a += part[2 * k]; b += part[2 * k + 1]; }
+  a = warp_sum(a); b = warp_sum(b);
+  const int w = threadIdx.x >> 5, l = threadIdx.x & 31;
+  if (l == 0) { red[0][w] = a; red[1][w] = b; }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    float ta = 0.f, tb = 0.f;
+    for (int k = 0; k < 8; ++k) { ta += red[0][k]; tb += red[1][k]; }
+    norms[2 * s] = ta;
+    norms[2 * s + 1] = tb;
   }
 }
 
@@ -206,7 +233,7 @@ extern "C" int passl_b200_sgd_momentum(float* p, const float* g, float* v, void*
   return PB_OK;
 }
 
-// norms: fp32 [2*num_segments] scratch (zeroed here); block_seg: int32 [ceil(n/1024)]; seg_wd: fp32 [num_segments]
+// norms: fp32 [2*num_segments] scratch (written here); block_seg: int32 [ceil(n/1024)]; seg_wd: fp32 [num_segments]
 extern "C" int passl_b200_lars_momentum(float* p, const float* g, float* v, void* p_bf16, const int* block_seg,
                                         const float* seg_wd, float* norms, int num_segments, float lr, float momentum,
                                         float lars_coeff, float eps, float grad_scale, const float* ctrl, long long n,
@@ -214,9 +241,21 @@ extern "C" int passl_b200_lars_momentum(float* p, const float* g, float* v, void
   if (n <= 0) return PB_OK;
   if (n % OPT_BLOCK) return PB_ERR_BAD_ARG;
   cudaStream_t st = (cudaStream_t)stream;
-  PB_CUDA_CHECK(cudaMemsetAsync(norms, 0, (size_t)num_segments * 8, st));
-  seg_sqnorm_kernel<<<opt_blocks(n), 256, 0, st>>>(p, g, block_seg, norms, grad_scale, n);
-  PB_LAUNCH_CHECK();
+  const int nblocks = opt_blocks(n);
+  float* part = nullptr;
+  int rc = splitk_scratch(&part, (size_t)nblocks * 2, st);
+  if (rc) return rc;
+  seg_sqnorm_kernel<<<nblocks, 256, 0, st>>>(p, g, part, grad_scale, n);
+  passl_b200_launch_counter_add(1);
+  cudaError_t launched = cudaGetLastError();
+  if (launched == cudaSuccess) {
+    seg_norm_finalize_kernel<<<num_segments, 256, 0, st>>>(part, block_seg, nblocks, norms);
+    passl_b200_launch_counter_add(1);
+    launched = cudaGetLastError();
+  }
+  rc = splitk_release(part, st);
+  if (launched != cudaSuccess) return (int)launched;
+  if (rc) return rc;
   lars_momentum_kernel<<<opt_blocks(n), 256, 0, st>>>(p, g, v, reinterpret_cast<__nv_bfloat16*>(p_bf16), block_seg, norms, seg_wd,
                                                       lr, momentum, lars_coeff, eps, grad_scale, ctrl, n);
   PB_LAUNCH_CHECK();

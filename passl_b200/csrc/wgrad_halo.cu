@@ -11,7 +11,7 @@
 //   warp 0 : TMA producer   dy box {64 co, 16, 8, 1} x 2,  x box {64 ci, 18, 10, 1}  (OOB zero fill = conv padding / ragged tiles)
 //   warp 1 : MMA issuer     per tap (r, s), per tile row h: A = dy rows [16h, 16h+16) (MN-major, two 64-channel atoms),
 //                           B = halo rows [(h+r)*18 + s, +16) (MN-major, start not 1024-aligned, base_offset 0)
-//   warps 2..5 : epilogue   tcgen05.ld -> red.global.add.f32 into dw (split-K across CTAs)
+//   warps 2..5 : epilogue   tcgen05.ld -> dw (one split) or this split's slice of the scratch that splitk_reduce adds into dw
 #include "common.cuh"
 #include "host_utils.h"
 #include "../../include/passl_b200.h"
@@ -33,6 +33,7 @@ constexpr int WH_SMEM = WH_STAGES * WH_STAGE_BYTES + 256 + 1024;   // >= WH_STAG
 struct WgradHaloParams {
   CUtensorMap dy_map, x_map;
   float* dw;
+  float* partial;        // splits > 1: split s stores its sums to partial + s * Cout * R * S * Cin, reduced in split order
   int N, H, W, Cin, Cout;
   int hb, wb;            // pixel tiles per image
   int k_total;           // N * hb * wb
@@ -173,13 +174,21 @@ __global__ void __launch_bounds__(192, 1) wgrad_halo_kernel(const __grid_constan
         for (int t = 0; t < ntap; ++t) {
           const int tap = tap0 + t;
           const int ci0 = ci_blk * 64 * p.cib;
-          float* dst = p.dw + ((size_t)co * (p.R * p.S) + tap) * p.Cin + ci0;
+          const size_t off = ((size_t)co * (p.R * p.S) + tap) * p.Cin + ci0;
+          float* part = p.partial ? p.partial + (size_t)(item % p.splits) * p.Cout * p.R * p.S * p.Cin + off : nullptr;
+          float* dst = p.dw + off;
 #pragma unroll 1
           for (int c = 0; c < 2 * p.cib; ++c) {
             uint32_t v[32];
             tmem_ld_32x32(tmem_base + ((q * 32u) << 16) + t * 64 * p.cib + c * 32, v);
             tmem_ld_wait();
-            if (row_ok) {
+            if (row_ok && part) {            // Cin % 64 == 0: whole 32-channel chunks, 16-byte aligned
+#pragma unroll
+              for (int j4 = 0; j4 < 8; ++j4)
+                *reinterpret_cast<float4*>(part + c * 32 + j4 * 4) =
+                    make_float4(__uint_as_float(v[j4 * 4]), __uint_as_float(v[j4 * 4 + 1]), __uint_as_float(v[j4 * 4 + 2]),
+                                __uint_as_float(v[j4 * 4 + 3]));
+            } else if (row_ok) {
 #pragma unroll
               for (int j = 0; j < 32; ++j)
                 if (ci0 + c * 32 + j < p.Cin) red_add_f32(dst + c * 32 + j, __uint_as_float(v[j]));
@@ -200,6 +209,11 @@ __global__ void __launch_bounds__(192, 1) wgrad_halo_kernel(const __grid_constan
     tmem_dealloc(tmem_base, 512);
   }
 }
+
+int splitk_scratch(float** out, size_t n_floats, cudaStream_t st);     // gemm_api.cu
+int splitk_release(float* ptr, cudaStream_t st);
+int splitk_reduce(float* out, const float* part, long long rows, long long cols, long long ld, long long stride, int splits,
+                  cudaStream_t st);
 
 int g_wgrad_halo_mode = 0;   // 0 auto (size heuristic), 1 always when the shape is supported, 2 never
 
@@ -255,8 +269,23 @@ int launch_wgrad_halo(const void* x, const void* dy, float* dw, int N, int H, in
   }
   const int items = base * splits;
   const int grid = items < num_sms() ? items : num_sms();
+  const long long wsize = (long long)Cout * R * S * Cin;
+  if (splits > 1) {
+    int rc = splitk_scratch(&p.partial, (size_t)splits * wsize, st);
+    if (rc) return rc;
+  }
   wgrad_halo_kernel<<<grid, 192, WH_SMEM, st>>>(p);
-  PB_LAUNCH_CHECK();
+  passl_b200_launch_counter_add(1);
+  const cudaError_t launched = cudaGetLastError();
+  if (launched != cudaSuccess) {
+    if (p.partial) splitk_release(p.partial, st);
+    return (int)launched;
+  }
+  if (splits > 1) {
+    int rc = splitk_reduce(dw, p.partial, Cout, R * S * Cin, R * S * Cin, wsize, splits, st);
+    int rc2 = splitk_release(p.partial, st);
+    return rc ? rc : rc2;
+  }
   return PB_OK;
 }
 

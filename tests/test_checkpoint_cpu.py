@@ -1,15 +1,13 @@
 """Paddle-checkpoint name / layout mapping (passl_b200/utils/checkpoint.py) checked against the reference classes themselves: the
-reference's ResNet-50 (resnetimagenet.py) and NonLinearNeckV1 (base_neck.py) are constructed over the paddle shim — no weights
-needed, only their parameter / buffer names and shapes — and must equal what `moco_to_paddle` emits."""
-import importlib
+reference's ResNet-50 (resnetimagenet.py) and NonLinearNeckV1 (base_neck.py) were constructed over the paddle shim — no weights
+needed, only their parameter / buffer names and shapes, stored in tests/golden/reference_checkpoint_names.npz by
+tests/golden/make_golden_checkpoint.py — and must equal what `moco_to_paddle` emits."""
 import os
-import sys
 
 import numpy as np
 import pytest
 import torch
 
-REF = "/root/reference"
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 
@@ -44,40 +42,14 @@ def test_roundtrip_and_file_container(tmp_path):
             assert torch.equal(sa[k], sb[k]), k
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="needs the reference tree (build container only)")
+def _ref_names(group):
+    """{name: shape} of one model's state_dict as the reference classes build it (tests/golden/make_golden_checkpoint.py)."""
+    G = np.load(os.path.join(HERE, "golden", "reference_checkpoint_names.npz"))
+    return {k[len(group) + 1:]: tuple(int(d) for d in G[k]) for k in G.files if k.startswith(group + ":")}, G
+
+
 def test_names_and_shapes_equal_the_reference_classes():
-    sys.path.insert(0, os.path.join(HERE, "golden"))
-    import make_golden
-    import make_golden_models as M
-    import paddle_shim  # noqa: F401
-    make_golden.setup()
-    M.extend_shim()
-    nn = sys.modules["paddle.nn"]
-
-    class Conv2D(nn.Layer):
-        def __init__(self, i, o, kernel_size, stride=1, padding=0, dilation=1, groups=1, bias_attr=None, **kw):
-            super().__init__()
-            self.weight = torch.nn.Parameter(torch.zeros(o, i, kernel_size, kernel_size))
-
-    class BatchNorm2D(nn.Layer):
-        def __init__(self, c, **kw):
-            super().__init__()
-            self.weight, self.bias = torch.nn.Parameter(torch.ones(c)), torch.nn.Parameter(torch.zeros(c))
-            self.register_buffer("_mean", torch.zeros(c))
-            self.register_buffer("_variance", torch.ones(c))
-
-    class MaxPool2D(nn.Layer):
-        def __init__(self, *a, **k):
-            super().__init__()
-    nn.Conv2D, nn.BatchNorm2D, nn.MaxPool2D = Conv2D, BatchNorm2D, MaxPool2D
-    rn = importlib.import_module("passl_v110.modeling.backbones.resnetimagenet")
-    necks = importlib.import_module("passl_v110.modeling.necks.base_neck")
-    ref_backbone = rn.ResNet(rn.BottleneckBlock, 50, num_classes=0, with_pool=False)
-    ref_neck = necks.NonLinearNeckV1(in_channels=2048, hid_channels=2048, out_channels=128)
-    want = {}
-    for pre, mod in (("encoder_q.0.", ref_backbone), ("encoder_q.1.", ref_neck)):
-        for k, v in mod.state_dict().items():
-            want[pre + k] = tuple(v.shape)
+    want, _ = _ref_names("moco")
     from passl_b200.utils import checkpoint as C
     got = {k: tuple(v.shape) for k, v in C.moco_to_paddle(_model()).items() if k.startswith("encoder_q.")}
     assert set(got) == set(want), (sorted(set(want) - set(got))[:5], sorted(set(got) - set(want))[:5])
@@ -165,66 +137,17 @@ def test_mocov3_roundtrip(tmp_path, literal):
     assert same != literal and ("momentum_predictor.fcs.0.weight" in sa) == literal
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="needs the reference tree (build container only)")
 def test_mocov3_names_and_shapes_equal_the_reference_class():
-    """passl/models/mocov3.py MoCoV3Pretrain constructed over the paddle shim (no weights needed): its state_dict keys and shapes,
-    including the CosineEMA wrapper's `momentum_encoder.model.{0,1}.*` / `steps`, must equal what mocov3_to_paddle emits."""
-    import functools
-    import types
-    sys.path.insert(0, GOLD)
-    import make_golden
-    import make_golden_models as M
-    import paddle_shim  # noqa: F401
-    make_golden.setup()
-    M.extend_shim()
-    import paddle
-    nn = sys.modules["paddle.nn"]
-    paddle.meshgrid = lambda *xs: torch.meshgrid(*xs, indexing="ij")
-    paddle.sin, paddle.cos = torch.sin, torch.cos
-
-    class Conv2D(nn.Layer):
-        def __init__(self, i, o, kernel_size, stride=1, padding=0, bias_attr=None, **kw):
-            super().__init__()
-            k = kernel_size if isinstance(kernel_size, (tuple, list)) else (kernel_size, kernel_size)
-            self.weight = torch.nn.Parameter(torch.zeros(o, i, k[0], k[1]))
-            self.bias = None if bias_attr is False else torch.nn.Parameter(torch.zeros(o))
-
-    class BatchNorm1D(nn.Layer):                 # Paddle keeps (frozen) weight / bias entries when weight_attr / bias_attr are False
-        def __init__(self, c, weight_attr=None, bias_attr=None, **kw):
-            super().__init__()
-            self.weight, self.bias = torch.nn.Parameter(torch.ones(c)), torch.nn.Parameter(torch.zeros(c))
-            self.register_buffer("_mean", torch.zeros(c))
-            self.register_buffer("_variance", torch.ones(c))
-    saved = {k: getattr(nn, k, None) for k in ("Conv2D", "BatchNorm1D", "LayerList")}
-    nn.Conv2D, nn.BatchNorm1D, nn.LayerList = Conv2D, BatchNorm1D, torch.nn.ModuleList
-    torch.Tensor._share_buffer_to = lambda self, other: None
-    torch.Tensor.set_value = lambda self, v: self.data.copy_(v)
-    nn.Layer.create_parameter = lambda self, shape, **kw: torch.nn.Parameter(torch.zeros(tuple(shape)), requires_grad=False)
-    nn.Layer.named_sublayers = lambda self: self.named_modules()
-
-    class _NoInit(types.ModuleType):
-        def __getattr__(self, n):
-            return lambda *a, **k: None
-    try:
-        vt = importlib.import_module("passl.models.vision_transformer")
-        vt.init = _NoInit("init")
-        mv = importlib.import_module("passl.models.mocov3")
-        mv.init = _NoInit("init")
-        ref = mv.MoCoV3Pretrain(functools.partial(mv.MoCoV3ViT, img_size=32, patch_size=8, embed_dim=64, depth=1, num_heads=2,
-                                                  mlp_ratio=4, qkv_bias=True), dim=32, mlp_dim=48)
-        want = {k: tuple(v.shape) for k, v in ref.state_dict().items()}
-        ref_pos = ref.base_encoder.pos_embed.detach().numpy()
-    finally:
-        for k, v in saved.items():
-            if v is not None:
-                setattr(nn, k, v)
+    """passl/models/mocov3.py MoCoV3Pretrain (no weights needed): its state_dict keys and shapes, including the CosineEMA
+    wrapper's `momentum_encoder.model.{0,1}.*` / `steps`, must equal what mocov3_to_paddle emits."""
+    want, G = _ref_names("mocov3")
     from passl_b200.utils import checkpoint as C
     ours = _small_mocov3()
     got = {k: tuple(v.shape) for k, v in C.mocov3_to_paddle(ours).items()}
     assert set(got) == set(want), (sorted(set(want) - set(got))[:5], sorted(set(got) - set(want))[:5])
     for k in want:
         assert got[k] == want[k], (k, got[k], want[k])
-    assert np.abs(ours.base_encoder.vit.pos_embed.numpy() - ref_pos).max() < 1e-6      # the fixed table the reference builds
+    assert np.abs(ours.base_encoder.vit.pos_embed.numpy() - G["mocov3_pos"]).max() < 1e-6      # the fixed table the reference builds
 
 
 def test_dispatch_covers_every_model_family():

@@ -217,3 +217,28 @@ def test_stem_wgrad_through_halo_kernel():
     dw_ref = wr.grad.permute(0, 2, 3, 1).reshape(64, 147)
     _check(dw_halo[:, :147], dw_ref, "stem wgrad halo", rel=1e-2)
     _check(dw_generic[:, :147], dw_ref, "stem wgrad generic", rel=1e-2)
+
+
+@pytest.mark.parametrize("case,halo_mode", [((64, 56, 56, 64, 256, 1, 1, 0), 0), ((64, 28, 28, 128, 128, 3, 1, 1), 1),
+                                            ((64, 28, 28, 128, 128, 3, 1, 1), 2), ((32, 28, 28, 128, 256, 3, 2, 1), 0)])
+def test_wgrad_split_k_is_bitwise_reproducible(case, halo_mode):
+    """Split-K weight gradients sum their slices in a fixed order: two launches on the same operands, accumulating into the same
+    starting values, give the same bits.  Cases: the 1x1 GEMM, the 3x3 halo-tile kernel (forced, mode 1), the generic 3x3 kernel
+    (halo off, mode 2) and the generic stride-2 kernel."""
+    from passl_b200 import _lib
+    from passl_b200 import kernels as K
+    N, H, W, Cin, Cout, R, stride, pad = case
+    torch.manual_seed(0)
+    Ho = (H + 2 * pad - R) // stride + 1
+    x = torch.randn(N, H, W, Cin, device="cuda").bfloat16()
+    dy = torch.randn(N, Ho, Ho, Cout, device="cuda").bfloat16()
+    base = torch.randn(Cout, R, R, Cin, device="cuda")
+    a, b = base.clone(), base.clone()
+    _lib.load().passl_b200_wgrad_halo_mode(halo_mode)
+    try:
+        K.conv2d_wgrad(x, dy, (Cout, R, R, Cin), stride=stride, pad=pad, out=a, accumulate=True)
+        K.conv2d_wgrad(x, dy, (Cout, R, R, Cin), stride=stride, pad=pad, out=b, accumulate=True)
+        torch.cuda.synchronize()
+    finally:
+        _lib.load().passl_b200_wgrad_halo_mode(0)
+    assert torch.equal(a, b)

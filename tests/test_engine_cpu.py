@@ -181,3 +181,25 @@ def test_bench_prints_exactly_one_json_line_on_stdout():
     assert len(lines) == 1, r.stdout
     d = json.loads(lines[0])
     assert d["impl"] == "reference" and "unavailable" in d
+
+
+def test_bench_dump_outputs_is_seeded_and_bounded(tmp_path):
+    """--dump-outputs writes loss / params / grads as float32; a buffer longer than DUMP_SAMPLE is sampled at the same positions
+    in every run (the master and gradient buffers at identical indices)."""
+    import types
+    import bench
+    n = bench.DUMP_SAMPLE + 12345
+    master = torch.arange(n, dtype=torch.float32)
+    store = types.SimpleNamespace(numel=n, master=master, grad=-master)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), torch.tensor([2.5]), store)
+    got = {f: np.load(tmp_path / "a" / (f + ".npy")) for f in ("loss", "params", "grads")}
+    assert all(v.dtype == np.float32 for v in got.values())
+    assert got["loss"].shape == () and float(got["loss"]) == 2.5
+    p = got["params"]
+    assert p.shape == (bench.DUMP_SAMPLE,) and np.all(np.diff(p) > 0) and p[-1] < n
+    assert np.array_equal(got["grads"], -p)
+    assert all(np.array_equal(v, np.load(tmp_path / "b" / (f + ".npy"))) for f, v in got.items())
+    small = types.SimpleNamespace(numel=5, master=master[:5], grad=master[:5])
+    bench.dump_outputs(str(tmp_path / "c"), torch.tensor(1.0), small)
+    assert np.array_equal(np.load(tmp_path / "c" / "params.npy"), master[:5].numpy())
