@@ -6,17 +6,10 @@
 // Input is the packed output of the qkv Linear, qkv[b][n][s][h][e] (s = 0/1/2 for q/k/v) — exactly the reference's
 // reshape [B,N,3,H,d] (vision_transformer.py:144-146) — read in place through a 4-D TMA tensor map (no permute pass).
 // Output O[b][n][h][e] = [T, H*d] (the layout the proj Linear consumes) + LSE[b][h][n] (natural log) for the backward.
-//
-// One CTA (160 threads) per SM loops over (b, h) work items; the whole K / V of a head sits in shared memory:
-//   warp 4 lane 0 : TMA loads of Q (128-row blocks), K, V; issues MMA1  S[128 x NKP] = Q_blk . K^T      (K = d)
-//                                                          and MMA2  O[128 x d]   = P . V          (K = NKP keys)
-//   warps 0..3    : one query row per thread: tcgen05.ld S from TMEM (2 passes: max, exp2+sum), write P (bf16) into
-//                   shared memory in the SWIZZLE_128B K-major layout the MMA reads, then normalise O out of TMEM.
 #include "common.cuh"
 #include "host_utils.h"
 #include "../../include/passl_b200.h"
 
-#include <stdlib.h>
 #include <string.h>
 
 namespace pb {
@@ -36,188 +29,9 @@ struct AttnParams {
   float scale;
 };
 
-__global__ void __launch_bounds__(160, 1) attn_fwd_kernel(const __grid_constant__ AttnParams p) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  const int rowB = p.d * 2;                         // bytes per Q/K/V row (128 or 64)
-  const uint32_t lt = (p.d == 64) ? 2u : 4u;        // SWIZZLE_128B / SWIZZLE_64B
-  const uint32_t sbo = 8u * rowB;                   // 8-row atom stride
-  uint8_t* q_s = smem;                              // [256][rowB]
-  uint8_t* k_s = q_s + 256 * rowB;                  // [256][rowB]
-  uint8_t* v_s = k_s + 256 * rowB;                  // [256][rowB]
-  uint8_t* p_s = v_s + 256 * rowB;                  // 4 chunks x [128][128 B]  (64 KB)
-  uint64_t* bars = reinterpret_cast<uint64_t*>(p_s + 4 * 128 * 128);
-  uint64_t* load_full = bars;      // tx
-  uint64_t* s_full = bars + 1;     // MMA1 commit
-  uint64_t* p_full = bars + 2;     // 4 warp arrivals
-  uint64_t* o_full = bars + 3;     // MMA2 commit
-  uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(bars + 4);
-
-  const uint32_t warp = warp_id(), lane = lane_id();
-  if (warp == 4 && lane == 0) {
-    tma_prefetch_desc(&p.qkv_map);
-    tma_prefetch_desc(&p.kv_map);
-    mbar_init(load_full, 1);
-    mbar_init(s_full, 1);
-    mbar_init(p_full, 4);
-    mbar_init(o_full, 1);
-    fence_barrier_init();
-  }
-  if (warp == 0) tmem_alloc(tmem_ptr, 512);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_ptr;
-  const uint32_t tm_s = tmem_base;          // S accumulator: columns [0, 256)
-  const uint32_t tm_o = tmem_base + 256;    // O accumulator: columns [256, 256 + d)
-
-  const int items = p.B * p.H;
-  uint32_t ph_load = 0, ph_s = 0, ph_p = 0, ph_o = 0;
-
-  if (warp == 4) {
-    {   // warp-uniform control loop; TMA / tcgen05 issue elect-predicated
-      const uint32_t idesc1 = make_idesc_bf16(128, p.NKP, false, false);
-      const uint32_t idesc2 = make_idesc_bf16(128, p.d, false, true);
-      for (int item = blockIdx.x; item < items; item += gridDim.x) {
-        const int b = item / p.H, h = item - b * p.H;
-        // all MMAs of the previous item have completed (we waited on its last o_full below) -> smem reusable
-        if (elect_one()) {
-          mbar_arrive_expect_tx(load_full, (uint32_t)((p.mblocks * 128 + 2 * p.NKP) * rowB));
-          for (int mb = 0; mb < p.mblocks; ++mb) tma_load_4d(q_s + mb * 128 * rowB, &p.qkv_map, load_full, 0, h, mb * 128, b);
-          tma_load_4d(k_s, &p.kv_map, load_full, 0, p.H + h, 0, b);
-          tma_load_4d(v_s, &p.kv_map, load_full, 0, 2 * p.H + h, 0, b);
-        }
-        __syncwarp();
-        mbar_wait(load_full, ph_load); ph_load ^= 1;
-        tc_fence_after();
-        for (int mb = 0; mb < p.mblocks; ++mb) {
-          // MMA1: S = Q_mb K^T
-          const uint32_t qa = smem_u32(q_s + mb * 128 * rowB), ka = smem_u32(k_s);
-          if (elect_one()) {
-            for (int k = 0; k < p.d / 16; ++k)
-              umma_bf16(tm_s, make_smem_desc(qa + k * 32, 16, sbo, lt), make_smem_desc(ka + k * 32, 16, sbo, lt), idesc1, k > 0);
-            umma_commit(s_full);
-          }
-          __syncwarp();
-          // MMA2: O = P V   (after the softmax warps published P)
-          mbar_wait(p_full, ph_p); ph_p ^= 1;
-          // o_full of the previous block has necessarily completed here (the softmax warps consumed it before
-          // publishing this P): consume the phase now so this thread never lags the barrier by two phases.
-          if (mb > 0) { mbar_wait(o_full, ph_o); ph_o ^= 1; }
-          tc_fence_after();
-          const uint32_t pa = smem_u32(p_s), va = smem_u32(v_s);
-          if (elect_one()) {
-            for (int k = 0; k < p.NKP / 16; ++k) {
-              uint64_t da = make_smem_desc_sw128(pa + (k >> 2) * (128 * 128) + (k & 3) * 32, 16, 1024);
-              uint64_t db = make_smem_desc(va + k * 16 * rowB, 0, sbo, lt);   // MN-major: 16 keys = 2 atoms of 8 rows
-              umma_bf16(tm_o, da, db, idesc2, k > 0);
-            }
-            umma_commit(o_full);
-          }
-          __syncwarp();
-        }
-        // wait until the last MMA2 of this item has retired before the next item's TMA overwrites smem
-        mbar_wait(o_full, ph_o); ph_o ^= 1;
-      }
-    }
-  } else {
-    // ---------------- softmax / epilogue warps (0..3): thread = query row ----------------
-    const uint32_t q4 = warp;                         // TMEM lane quarter == warp id (0..3)
-    const int r = q4 * 32 + lane;                     // row within the 128-row block
-    const float c2 = p.scale * kAttnLog2e;
-    for (int item = blockIdx.x; item < items; item += gridDim.x) {
-      const int b = item / p.H, h = item - b * p.H;
-      for (int mb = 0; mb < p.mblocks; ++mb) {
-        const int row = mb * 128 + r;                 // query index
-        const bool row_ok = row < p.N;
-        const int jmax = p.causal ? (row + 1 < p.N ? row + 1 : p.N) : p.N;   // valid keys: j < jmax
-        mbar_wait(s_full, ph_s); ph_s ^= 1;
-        tc_fence_after();
-        const uint32_t ts = tm_s + ((q4 * 32u) << 16);
-        // pass 1: row maximum (log2 domain)
-        float m = -INFINITY;
-        for (int c = 0; c < p.NKP / 32; ++c) {
-          uint32_t v[32];
-          tmem_ld_32x32(ts + c * 32, v);
-          tmem_ld_wait();
-#pragma unroll
-          for (int j = 0; j < 32; ++j)
-            if (c * 32 + j < jmax) m = fmaxf(m, __uint_as_float(v[j]) * c2);
-        }
-        if (!row_ok || m == -INFINITY) m = 0.f;
-        // pass 2: p = exp2(y - m), row sum, P -> smem (bf16, SWIZZLE_128B K-major: chunk of 64 keys = [128 rows][128 B])
-        float l = 0.f, l_exact = 0.f;
-        for (int c = 0; c < p.NKP / 32; ++c) {
-          uint32_t v[32];
-          tmem_ld_32x32(ts + c * 32, v);
-          tmem_ld_wait();
-          float e[32];
-#pragma unroll
-          for (int j = 0; j < 32; ++j) {
-            const float pj = (c * 32 + j < jmax) ? exp2f(__uint_as_float(v[j]) * c2 - m) : 0.f;
-            // the tensor core multiplies the bf16-rounded probability: normalise O by the sum of the same rounded values,
-            // but report the exact log-sum-exp (the backward recomputes P from it)
-            e[j] = __bfloat162float(__float2bfloat16_rn(pj));
-            l += e[j];
-            l_exact += pj;
-          }
-          const int chunk = (c * 32) >> 6;
-          uint8_t* base = p_s + chunk * (128 * 128) + (r >> 3) * 1024 + (r & 7) * 128;
-#pragma unroll
-          for (int g = 0; g < 4; ++g) {
-            const int j8 = ((c * 32) & 63) + g * 8;                // key offset within the 64-key chunk
-            uint4 u;
-            u.x = pack_bf16x2(e[g * 8 + 0], e[g * 8 + 1]);
-            u.y = pack_bf16x2(e[g * 8 + 2], e[g * 8 + 3]);
-            u.z = pack_bf16x2(e[g * 8 + 4], e[g * 8 + 5]);
-            u.w = pack_bf16x2(e[g * 8 + 6], e[g * 8 + 7]);
-            *reinterpret_cast<uint4*>(base + ((((j8 >> 3) ^ (r & 7)) & 7) << 4)) = u;
-          }
-        }
-        tc_fence_before();
-        fence_proxy_async_smem();      // generic-proxy smem writes -> visible to the tensor core (async proxy)
-        __syncwarp();
-        if (lane == 0) mbar_arrive(p_full);
-        // epilogue: O / l
-        mbar_wait(o_full, ph_o); ph_o ^= 1;
-        tc_fence_after();
-        const uint32_t to = tm_o + ((q4 * 32u) << 16);
-        const float inv = (l > 0.f) ? 1.f / l : 0.f;
-        __nv_bfloat16* op = p.out + (((size_t)b * p.N + row) * p.H + h) * p.d;
-        for (int c = 0; c < p.d / 32; ++c) {
-          uint32_t v[32];
-          tmem_ld_32x32(to + c * 32, v);
-          tmem_ld_wait();
-          if (row_ok) {
-#pragma unroll
-            for (int g = 0; g < 4; ++g) {
-              uint4 u;
-              u.x = pack_bf16x2(__uint_as_float(v[g * 8 + 0]) * inv, __uint_as_float(v[g * 8 + 1]) * inv);
-              u.y = pack_bf16x2(__uint_as_float(v[g * 8 + 2]) * inv, __uint_as_float(v[g * 8 + 3]) * inv);
-              u.z = pack_bf16x2(__uint_as_float(v[g * 8 + 4]) * inv, __uint_as_float(v[g * 8 + 5]) * inv);
-              u.w = pack_bf16x2(__uint_as_float(v[g * 8 + 6]) * inv, __uint_as_float(v[g * 8 + 7]) * inv);
-              *reinterpret_cast<uint4*>(op + c * 32 + g * 8) = u;
-            }
-          }
-        }
-        if (row_ok) p.lse[((size_t)b * p.H + h) * p.N + row] = (m + log2f(l_exact)) * kAttnLn2;
-        tc_fence_before();
-      }
-    }
-  }
-
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 0) {
-    __syncwarp();
-    tmem_dealloc(tmem_base, 512);
-  }
-}
-
 // ======================================================================================================================
-// Forward, pipelined (round 2).  The round-1 kernel above ran load -> QK^T -> softmax -> PV -> epilogue strictly in sequence per
-// (batch, head): 114 TF/s at B=512, N=197, d=64.  Here one CTA (320 threads) keeps TWO work items (128 query rows of one head)
-// in flight:
+// Forward, pipelined: load -> QK^T -> softmax -> PV -> epilogue strictly in sequence per (batch, head) ran at 114 TF/s at B=512,
+// N=197, d=64.  One CTA (320 threads) keeps TWO work items (128 query rows of one head) in flight:
 //   warp 0      : TMA producer — K / V of a head once (2-stage ring, shared by the head's query blocks), Q blocks (3-stage ring)
 //   warp 1      : MMA issuer — S = Q K^T of item i, then O = P V of item i-1 (P read from TMEM as the A operand, V from shared
 //                 memory as an MN-major B operand), so the tensor pipe works on one item while the SFUs work on the other
@@ -488,31 +302,17 @@ extern "C" int passl_b200_attention_fwd(const void* qkv, void* out, float* lse, 
   p.mblocks = (N + 127) / 128;
   int rc = attn_make_maps(p, qkv);
   if (rc) return rc;
-  int grid = B * H < num_sms() ? B * H : num_sms();
-  static int use_v1 = -1;
-  if (use_v1 < 0) use_v1 = getenv("PASSL_B200_ATTN_V1") ? 1 : 0;      // round-1 serial kernel, kept for A/B timing
-  if (!use_v1) {
-    const int kvB = ((p.NKP * d * 2) + 1023) & ~1023;
-    const int smem2 = 3 * 128 * d * 2 + 4 * kvB + 256 + 1024;
-    static bool attr2 = false;
-    if (!attr2) {
-      PB_CUDA_CHECK(cudaFuncSetAttribute(attn_fwd2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (3 * 128 + 4 * 256) * 128 + 256 + 1024));
-      attr2 = true;
-    }
-    // short sequences: two CTAs per SM (shared memory and the 256-column TMEM allocation allow it) -> four items in flight per SM
-    const int per_sm = (p.NKP <= 64 && smem2 <= 100 * 1024) ? 2 : 1;
-    grid = B * H < num_sms() * per_sm ? B * H : num_sms() * per_sm;
-    attn_fwd2_kernel<<<grid, 320, smem2, (cudaStream_t)stream>>>(p);
-    PB_LAUNCH_CHECK();
-    return PB_OK;
-  }
-  const int smem = 3 * 256 * d * 2 + 4 * 128 * 128 + 256 + 1024;
+  const int kvB = ((p.NKP * d * 2) + 1023) & ~1023;
+  const int smem = 3 * 128 * d * 2 + 4 * kvB + 256 + 1024;
   static bool attr = false;
   if (!attr) {
-    PB_CUDA_CHECK(cudaFuncSetAttribute(attn_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 3 * 256 * 128 + 4 * 128 * 128 + 256 + 1024));
+    PB_CUDA_CHECK(cudaFuncSetAttribute(attn_fwd2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (3 * 128 + 4 * 256) * 128 + 256 + 1024));
     attr = true;
   }
-  attn_fwd_kernel<<<grid, 160, smem, (cudaStream_t)stream>>>(p);
+  // short sequences: two CTAs per SM (shared memory and the 256-column TMEM allocation allow it) -> four items in flight per SM
+  const int per_sm = (p.NKP <= 64 && smem <= 100 * 1024) ? 2 : 1;
+  const int grid = B * H < num_sms() * per_sm ? B * H : num_sms() * per_sm;
+  attn_fwd2_kernel<<<grid, 320, smem, (cudaStream_t)stream>>>(p);
   PB_LAUNCH_CHECK();
   return PB_OK;
 }

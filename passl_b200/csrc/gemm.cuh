@@ -86,7 +86,6 @@ struct GemmParams {
   // squares), zero-initialised by the host; row 4*b + q is only touched by the two epilogue warps of lane quarter q of CTA b, on
   // disjoint columns -> no atomics, deterministic per grid
   float* col_sum;
-  float* col_sqsum;     // unused (kept for ABI stability of the struct users)
   // residual through the tensor pipe: when res_iters > 0 the producer appends res_iters (= 128 / 64) pipeline iterations per tile
   // that load an identity slice as A and the residual tile (MN-major) as B, so that D += I * R — the residual is prefetched as
   // deep as the operands (a register prefetch in the epilogue cannot cover the ~4 us DRAM latency of a saturated HBM)
@@ -99,7 +98,6 @@ struct GemmParams {
   CUtensorMap tile_map;
   int tile_prefetch;
   int halo_dh0, halo_dw0;   // HALO variant: smallest row / column shift over the taps = origin of the halo box relative to the tile
-  int dbg;              // developer perf experiments (PASSL_B200_EPI_DEBUG): 1 skip stats, 2 skip global stores, 4 skip staging
 };
 
 // EW = number of epilogue warps: 8 (two per TMEM lane quarter), or 16 for the epilogue-bound linear launches (GELU / gate
@@ -817,7 +815,7 @@ __global__ void __launch_bounds__(64 + 32 * EW, 1) gemm_tcgen05_kernel(const __g
     const uint32_t bias_u32 = smem_u32(epi_stage + EW * 32 * kEpiStride + e * (4 * 32 * 4));
     const uint32_t stg_u32 = smem_u32(stg);
     const bool staged = !p.out_fp32;
-    const bool do_stats = staged && p.col_sum != nullptr && !(p.dbg & 1);
+    const bool do_stats = staged && p.col_sum != nullptr;
     // BatchNorm statistics: per-warp register accumulators (lanes 0..15 own the column pairs of each of the warp's chunks), kept
     // across tiles while the CTA stays on one column block and folded into the warp's own global partial row (row = CTA*4 + lane
     // quarter; the two warps of a quarter own disjoint columns) — no atomics, no barriers
@@ -1085,7 +1083,6 @@ __global__ void __launch_bounds__(64 + 32 * EW, 1) gemm_tcgen05_kernel(const __g
 #pragma unroll
           for (int i = 0; i < 4; ++i) rr[i] = rn[i];          // the tile prefetched for this warp's next chunk
         }
-        if (p.dbg & 4) continue;
 #pragma unroll
         for (int j8 = 0; j8 < 4; ++j8) {
           uint4 u = make_uint4(0u, 0u, 0u, 0u);                 // rows outside the tensor contribute zeros to the statistics
@@ -1117,12 +1114,10 @@ __global__ void __launch_bounds__(64 + 32 * EW, 1) gemm_tcgen05_kernel(const __g
             if (i == ci) { sacc[i][0] += sa; sacc[i][1] += sb; sacc[i][2] += qa; sacc[i][3] += qb; }
         }
         __nv_bfloat16* outp = reinterpret_cast<__nv_bfloat16*>(p.out);
-        if (!(p.dbg & 2)) {
 #pragma unroll
-          for (int i = 0; i < 4; ++i) {
-            if (ro4[i] >= 0 && col_ok)
-              *reinterpret_cast<uint4*>(outp + ro4[i] + oc0 + cch * 8) = ld_shared_v4(stg_u32 + (i * 8 + crow) * kEpiStride + cch * 16);
-          }
+        for (int i = 0; i < 4; ++i) {
+          if (ro4[i] >= 0 && col_ok)
+            *reinterpret_cast<uint4*>(outp + ro4[i] + oc0 + cch * 8) = ld_shared_v4(stg_u32 + (i * 8 + crow) * kEpiStride + cch * 16);
         }
         __syncwarp();
       }

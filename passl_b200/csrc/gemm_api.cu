@@ -1,11 +1,11 @@
 // C-ABI launchers for the tcgen05 GEMM / implicit-GEMM convolution kernel (see gemm.cuh).
-#include <stdlib.h>
 #include "gemm.cuh"
 #include "host_utils.h"
 #include "../../include/passl_b200.h"
 
 #include <string.h>
 
+#include <functional>
 #include <mutex>
 
 namespace pb {
@@ -34,9 +34,7 @@ static int eye128_ptr(const void** out, cudaStream_t st) {
 // route the residual through the MMA when the epilogue semantics allow it (out = A.B + bias + residual, bf16, plain row-major)
 static int setup_residual_mma(GemmParams& p, const void* residual, long long ldc, cudaStream_t st) {
   p.res_iters = 0;
-  static int off = -1;
-  if (off < 0) { const char* e = getenv("PASSL_B200_NO_RES_MMA"); off = e ? atoi(e) : 0; }
-  if (off || !residual || p.out_fp32 || p.out_pixel || p.act != ACT_NONE || p.alpha != 1.f || p.aux || p.preact || p.splits != 1 ||
+  if (!residual || p.out_fp32 || p.out_pixel || p.act != ACT_NONE || p.alpha != 1.f || p.aux || p.preact || p.splits != 1 ||
       p.n_blocks_per_tap > 0 || (reinterpret_cast<uintptr_t>(residual) & 15))
     return PB_OK;
   const void* eye = nullptr;
@@ -69,9 +67,6 @@ static int launch_gemm_t(const GemmParams& p, cudaStream_t st) {
   int slots = num_sms() / CG;
   int grid = (tiles < slots ? tiles : slots) * CG;
   if (grid <= 0) return PB_OK;
-  static int dbg = -1;
-  if (dbg < 0) { const char* e = getenv("PASSL_B200_EPI_DEBUG"); dbg = e ? atoi(e) : 0; }
-  const_cast<GemmParams&>(p).dbg = dbg;
   if (p.col_sum) {
     if (p.out_fp32 || p.n_blocks_per_tap > 0 || p.splits != 1) return PB_ERR_UNSUPPORTED;
     PB_CUDA_CHECK(cudaMemsetAsync(p.col_sum, 0, (size_t)num_sms() * 4 * 2 * p.N * sizeof(float), st));
@@ -95,19 +90,12 @@ static int launch_gemm_t(const GemmParams& p, cudaStream_t st) {
   return PB_OK;
 }
 
-// CTA pairs (cta_group::2, gemm.cuh) for the big K-major-A tiles; PASSL_B200_GEMM_PAIR=0 keeps every launch single-CTA
-static bool pair_enabled() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("PASSL_B200_GEMM_PAIR"); v = (e && !atoi(e)) ? 0 : 1; }
-  return v != 0;
-}
+// CTA pairs (cta_group::2, gemm.cuh) for the big K-major-A tiles
 static bool pair_eligible(const GemmParams& p, int BN, int BK, bool a_mn) {
   // k_iters: a tile with a short K loop (1x1 convolutions on 64..256 channels) is bound by its epilogue / HBM, where the pair
-  // only couples two epilogues to one MMA stream (PASSL_B200_GEMM_PAIR_MINK overrides the threshold)
-  static int mink = -1;
-  if (mink < 0) { const char* e = getenv("PASSL_B200_GEMM_PAIR_MINK"); mink = e ? atoi(e) : 8; }
-  return pair_enabled() && BN == 256 && BK == 64 && !a_mn && p.res_iters == 0 && p.a.mode != OP_PATCH_MN && p.b.mode != OP_PATCH_MN &&
-         p.k_iters >= mink && (long long)((p.m_blocks + 1) / 2) * p.n_blocks * p.splits >= num_sms() / 2;
+  // only couples two epilogues to one MMA stream
+  return BN == 256 && BK == 64 && !a_mn && p.res_iters == 0 && p.a.mode != OP_PATCH_MN && p.b.mode != OP_PATCH_MN &&
+         p.k_iters >= 8 && (long long)((p.m_blocks + 1) / 2) * p.n_blocks * p.splits >= num_sms() / 2;
 }
 
 // Split-K partial sums are added in a fixed order so that a launch computes the same bits every run (float red.add in
@@ -167,8 +155,8 @@ __global__ void splitk_reduce_kernel(float* __restrict__ out, const float* __res
   }
 }
 
-int splitk_reduce(float* out, const float* part, long long rows, long long cols, long long ld, long long stride, int splits,
-                  cudaStream_t st) {
+static int splitk_reduce(float* out, const float* part, long long rows, long long cols, long long ld, long long stride, int splits,
+                         cudaStream_t st) {
   if (cols % 4 || ld % 4 || stride % 4 || rows * cols >= (1ll << 32)) return PB_ERR_UNSUPPORTED;
   const long long n = rows * cols / 4;
   const long long cap = (long long)num_sms() * 8;
@@ -178,18 +166,29 @@ int splitk_reduce(float* out, const float* part, long long rows, long long cols,
   return PB_OK;
 }
 
+// Runs launch(partial) with scratch for `splits` slices of rows x ld floats (slice s at partial + s * rows * ld, addressed like
+// out), adds the slices into out in split order and releases the scratch, also when the launch fails.
+int splitk_run(float* out, long long rows, long long cols, long long ld, int splits, cudaStream_t st,
+               const std::function<int(float*)>& launch) {
+  float* partial = nullptr;
+  int rc = splitk_scratch(&partial, (size_t)splits * rows * ld, st);
+  if (rc) return rc;
+  rc = launch(partial);
+  if (!rc) rc = splitk_reduce(out, partial, rows, cols, ld, rows * ld, splits, st);
+  const int rc2 = splitk_release(partial, st);
+  return rc ? rc : rc2;
+}
+
 static int launch_gemm(const GemmParams& p, int BN, int BK, bool a_mn, bool b_mn, cudaStream_t st, int epi = 0, int cg = 1,
                        bool halo = false, int ew = 8) {
   if (p.atomic_add && p.splits > 1 && !p.partial) {
     if (p.ldc % 4 || p.N % 4) return PB_ERR_UNSUPPORTED;
-    GemmParams q = p;
-    q.part_stride = (long long)p.M * p.ldc;
-    int rc = splitk_scratch(&q.partial, (size_t)p.splits * q.part_stride, st);
-    if (rc) return rc;
-    rc = launch_gemm(q, BN, BK, a_mn, b_mn, st, epi, cg, halo, ew);
-    if (!rc) rc = splitk_reduce(reinterpret_cast<float*>(p.out), q.partial, p.M, p.N, p.ldc, q.part_stride, p.splits, st);
-    int rc2 = splitk_release(q.partial, st);
-    return rc ? rc : rc2;
+    return splitk_run(reinterpret_cast<float*>(p.out), p.M, p.N, p.ldc, p.splits, st, [&](float* partial) {
+      GemmParams q = p;
+      q.partial = partial;
+      q.part_stride = (long long)p.M * p.ldc;
+      return launch_gemm(q, BN, BK, a_mn, b_mn, st, epi, cg, halo, ew);
+    });
   }
   if (ew == 16 && epi == 2 && cg == 1 && BN == 256 && BK == 64 && !a_mn && !b_mn && !halo)   // K-small 1x1 convolutions with statistics
     return launch_gemm_t<256, 64, false, false, 2, 1, false, 16>(p, st);
@@ -217,9 +216,13 @@ static int launch_gemm(const GemmParams& p, int BN, int BK, bool a_mn, bool b_mn
     if (epi == 1) return b_mn ? launch_gemm_t<256, 64, false, true, 1, 2>(p, st) : launch_gemm_t<256, 64, false, false, 1, 2>(p, st);
     return b_mn ? launch_gemm_t<256, 64, false, true, 0, 2>(p, st) : launch_gemm_t<256, 64, false, false, 0, 2>(p, st);
   }
+  if (BK == 128) {     // the generic convolution weight gradient (conv_wgrad_impl): BN 64 or 128
+    if (BN == 64) return launch_gemm_t<64, 128, true, true>(p, st);
+    if (BN == 128) return launch_gemm_t<128, 128, true, true>(p, st);
+    return PB_ERR_UNSUPPORTED;
+  }
 #define PB_DISPATCH(bn)                                                                 \
   if (BN == bn) {                                                                       \
-    if (BK == 128) return launch_gemm_t<bn, 128, true, true>(p, st);                    \
     if (epi == 2 && !a_mn && !b_mn) return launch_gemm_t<bn, 64, false, false, 2>(p, st); \
     if (epi == 1 && !a_mn && !b_mn) return launch_gemm_t<bn, 64, false, false, 1>(p, st); \
     if (epi == 1 && !a_mn && b_mn) return launch_gemm_t<bn, 64, false, true, 1>(p, st);   \
@@ -265,10 +268,10 @@ static int fill_mat_operand(GemmOperand& op, const void* base, bool mn_major, lo
 }
 
 static void set_epilogue(GemmParams& p, void* out, long long ldc, int out_fp32, int atomic_add, const float* bias,
-                         const void* residual, int act, float alpha, float* col_sum, float* col_sqsum) {
+                         const void* residual, int act, float alpha, float* col_sum) {
   p.out = out; p.ldc = ldc; p.out_fp32 = out_fp32; p.atomic_add = atomic_add;
   p.bias = bias; p.residual = reinterpret_cast<const __nv_bfloat16*>(residual);
-  p.act = act; p.alpha = alpha; p.col_sum = col_sum; p.col_sqsum = col_sqsum;
+  p.act = act; p.alpha = alpha; p.col_sum = col_sum;
 }
 
 // ---- patch geometry ------------------------------------------------------------------------
@@ -284,11 +287,8 @@ static void pick_patch(PatchGeom& g, int Nimg, int Ho, int Wo) {
 }
 
 // 3x3 (or any <= 3x3, stride 1) convolution through ONE halo box per channel chunk (gemm.cuh HALO): 16 x 8 pixel tiles of one image.
-// PASSL_B200_CONV_HALO=0 keeps the per-tap loads.
 static bool conv_halo_ok(int H, int W, int ntaps, const signed char* dh, const signed char* dw, int& dh0, int& dw0) {
-  static int en = -1;
-  if (en < 0) { const char* e = getenv("PASSL_B200_CONV_HALO"); en = (e && !atoi(e)) ? 0 : 1; }
-  if (!en || H < 12 || W < 8 || ntaps < 2) return false;
+  if (H < 12 || W < 8 || ntaps < 2) return false;
   int hmin = 127, hmax = -127, wmin = 127, wmax = -127;
   for (int t = 0; t < ntaps; ++t) {
     hmin = dh[t] < hmin ? dh[t] : hmin; hmax = dh[t] > hmax ? dh[t] : hmax;
@@ -308,9 +308,7 @@ static bool conv_halo_ok(int H, int W, int ntaps, const signed char* dh, const s
 // Returns the epilogue variant (1 plain, 2 with column statistics) or 0 when the pixel-addressed epilogue has to stay.
 static int halo_lean_epi(GemmParams& p, int BN, int cg, void* out, int N, int Ho, int Wo, int C, const void* residual, int act,
                          float* col_sum) {
-  static int en = -1;
-  if (en < 0) { const char* e = getenv("PASSL_B200_CONV_HALO_TMA_STORE"); en = (e && !atoi(e)) ? 0 : 1; }
-  if (!en || residual || act > ACT_RELU || (C % 8) || (reinterpret_cast<uintptr_t>(out) & 15)) return 0;
+  if (residual || act > ACT_RELU || (C % 8) || (reinterpret_cast<uintptr_t>(out) & 15)) return 0;
   if (!((BN == 64 && cg == 1) || BN == 256)) return 0;
   uint64_t dims[4] = {(uint64_t)C, (uint64_t)Wo, (uint64_t)Ho, (uint64_t)N};
   uint64_t str[3] = {(uint64_t)C * 2, (uint64_t)Wo * C * 2, (uint64_t)Ho * Wo * C * 2};
@@ -357,6 +355,42 @@ static int fill_patch_maps(GemmOperand& op, const void* base, int N, int H, int 
   return PB_OK;
 }
 
+// One implicit GEMM of a convolution (the forward, or one output-parity class of the data gradient).  Rows: the pixels of an
+// (OH / os) x (OW / os) grid per image, stored to NHWC out [N, OH, OW, cols] at (oh0 + os * h, ow0 + os * w).  A: NHWC src
+// [N, Hs, Ws, C] through the per-tap shifts the caller left in p.a.dh / dw / map (src_stride 2: parity maps).  B: wmat
+// [cols][ntaps * C].  A stride-1 convolution whose output has the extent of its input may take the HALO tiles; with a
+// residual only when halo_residual.
+static int conv_igemm(GemmParams& p, const void* src, int N, int Hs, int Ws, int C, int src_stride, int ntaps, const void* wmat,
+                      int cols, void* out, int OH, int OW, int os, int oh0, int ow0, const float* bias, const void* residual,
+                      int act, float* col_sum, bool halo_residual, cudaStream_t st) {
+  const int Hg = OH / os, Wg = OW / os;
+  const bool halo = src_stride == 1 && os == 1 && OH == Hs && OW == Ws && (halo_residual || !residual) &&
+                    conv_halo_ok(Hs, Ws, ntaps, p.a.dh, p.a.dw, p.halo_dh0, p.halo_dw0);
+  if (halo) halo_geom(p.geom, N, Hg, Wg);
+  else pick_patch(p.geom, N, Hg, Wg);
+  p.M = N * Hg * Wg; p.N = cols;
+  p.m_blocks = p.geom.nb * p.geom.hb * p.geom.wb;
+  const int BN = pick_bn(p.m_blocks, cols);
+  p.n_blocks = (cols + BN - 1) / BN;
+  p.splits = 1;
+  p.a.mode = OP_PATCH_K;
+  p.a.cchunks = C / 64;
+  p.a.ntaps = ntaps;
+  p.a.tx_bytes = p.geom.TN * p.geom.TH * p.geom.TW * 128;
+  int rc = halo ? fill_halo_map(p.a, src, N, Hs, Ws, C) : fill_patch_maps(p.a, src, N, Hs, Ws, C, src_stride, p.geom);
+  if (rc) return rc;
+  p.k_iters = ntaps * p.a.cchunks;
+  p.k_steps = 4;
+  // (CTA pairs on the 64-wide halo tiles were measured and dropped: 64 ch at 56x56 forward 453 -> 545 us, dgrad 427 -> 501 us)
+  const int cg = pair_eligible(p, BN, 64, false) ? 2 : 1;
+  rc = fill_mat_operand(p.b, wmat, false, cols, (long long)ntaps * C, (long long)ntaps * C, BN / cg, 64);
+  if (rc) return rc;
+  set_epilogue(p, out, cols, 0, 0, bias, residual, act, 1.f, col_sum);
+  p.out_pixel = 1; p.OH = OH; p.OW = OW; p.osh = os; p.osw = os; p.oh0 = oh0; p.ow0 = ow0;
+  const int hepi = halo ? halo_lean_epi(p, BN, cg, out, N, OH, OW, cols, residual, act, col_sum) : 0;
+  return launch_gemm(p, BN, 64, false, false, st, hepi, cg, halo);
+}
+
 }  // namespace pb
 
 using namespace pb;
@@ -395,7 +429,7 @@ extern "C" int passl_b200_gemm_bf16_ex(const void* A, const void* B, void* out, 
   // from L2 at full MMA rate (delivered: ~50), so they ran at 0.45-0.65 of a plain GEMM.  A CTA pair on a 256 x 256 tile needs half
   // of that per SM; the caller's split count is replaced by the one that minimises whole waves of num_sms / 2 clusters x item length.
   bool wgrad_pair = false;
-  if (a_mn_major && b_mn_major && out_fp32 && atomic_add && splits > 1 && N % 256 == 0 && M >= 256 && pair_enabled() && !bias && !residual && !aux) {
+  if (a_mn_major && b_mn_major && out_fp32 && atomic_add && splits > 1 && N % 256 == 0 && M >= 256 && !bias && !residual && !aux) {
     const int slots = num_sms() / 2;
     const int ptiles = ((p.m_blocks + 1) / 2) * (N / 256);
     // cost of a split count in K iterations: whole waves x (iterations per item + ~32 for the pipeline fill and the 128 KB of
@@ -418,18 +452,15 @@ extern "C" int passl_b200_gemm_bf16_ex(const void* A, const void* B, void* out, 
   // nor when a residual could ride the MMA of a short K loop instead of the epilogue (proj of ViT-B: 999 vs 917 TF/s)
   // GELU / gate launches: epilogue-bound.  With 8 epilogue warps a pair only couples two slow epilogues to one MMA stream (-5 %);
   // with 16 warps per CTA and K >= 768 the pair wins (fc2-dgrad + GELU' 817 -> 1011 TF/s, fc1 + GELU 1017 -> 1064 at the CLIP batch;
-  // K = 512: 798 -> 753, so those stay single).  PASSL_B200_GEMM_HEAVY_PAIR=0 / PASSL_B200_GEMM_EW16=0 switch the two off.
-  static int heavy_pair = -1, ew16 = -1;
-  if (heavy_pair < 0) { const char* e = getenv("PASSL_B200_GEMM_HEAVY_PAIR"); heavy_pair = (e && !atoi(e)) ? 0 : 1; }
-  if (ew16 < 0) { const char* e = getenv("PASSL_B200_GEMM_EW16"); ew16 = (e && !atoi(e)) ? 0 : 1; }
+  // K = 512: 798 -> 753, so those stay single).
   const bool heavy = act == ACT_GELU || act == ACT_QUICKGELU || (aux && aux_mode >= 2);
-  const bool heavy_pair_ok = heavy && heavy_pair && ew16 && K >= 768;
+  const bool heavy_pair_ok = heavy && K >= 768;
   const bool heavy_epi = heavy && !heavy_pair_ok;
   const bool short_k_residual = residual && K < 1536;
   const int cg = (wgrad_pair || (!heavy_epi && !short_k_residual && pair_eligible(p, BN, 64, a_mn_major != 0))) ? 2 : 1;
   r = fill_mat_operand(p.b, B, b_mn_major != 0, N, K, ldb, BN / cg, 64);
   if (r) return r;
-  set_epilogue(p, out, ldc, out_fp32, atomic_add, bias, residual, act, alpha, col_sum, col_sqsum);
+  set_epilogue(p, out, ldc, out_fp32, atomic_add, bias, residual, act, alpha, col_sum);
   p.aux = reinterpret_cast<const __nv_bfloat16*>(aux);
   p.aux_mode = aux_mode;
   p.preact = reinterpret_cast<__nv_bfloat16*>(preact_out);
@@ -439,12 +470,10 @@ extern "C" int passl_b200_gemm_bf16_ex(const void* A, const void* B, void* out, 
   }
   // linear-layer epilogue (EPI 1, TMA stores): plain row-major bf16 output, K-major A, no statistics / scaling, at most one
   // operand tile (gate operand or a residual that does not go through the MMA)
-  static int lean = -1;
-  if (lean < 0) { const char* e = getenv("PASSL_B200_GEMM_EPI0"); lean = (e && atoi(e)) ? 0 : 1; }
   int epi = 0;
   const bool res_in_epilogue = residual && p.res_iters == 0;
   const bool stats_ok = !col_sum || (!b_mn_major && act <= ACT_RELU && !preact_out && (!aux || aux_mode == 1));   // EPI 2
-  if (lean && !out_fp32 && !a_mn_major && stats_ok && alpha == 1.f && splits == 1 && !(aux && res_in_epilogue) &&
+  if (!out_fp32 && !a_mn_major && stats_ok && alpha == 1.f && splits == 1 && !(aux && res_in_epilogue) &&
       !((reinterpret_cast<uintptr_t>(aux) | reinterpret_cast<uintptr_t>(preact_out) | reinterpret_cast<uintptr_t>(residual)) & 15)) {
     uint64_t dims[2] = {(uint64_t)N, (uint64_t)M}, strides[1] = {(uint64_t)ldc * 2};
     uint32_t box[2] = {32, 32};
@@ -466,8 +495,8 @@ extern "C" int passl_b200_gemm_bf16_ex(const void* A, const void* B, void* out, 
   // 746 -> 783, K = 768: 940 -> 917), `profiles/r02_vit_gemm_probe_ew16.txt`
   // (also the 1x1 convolutions with BatchNorm statistics and a K loop of <= 4 iterations: one MMA group per tile, the epilogue is all
   // there is)
-  const bool use16 = ew16 && ((aux && aux_mode >= 2) || ((act == ACT_GELU || act == ACT_QUICKGELU) && (K < 768 || (heavy_pair_ok && cg == 2))) ||
-                              (epi == 2 && cg == 1 && p.k_iters <= 4));
+  const bool use16 = (aux && aux_mode >= 2) || ((act == ACT_GELU || act == ACT_QUICKGELU) && (K < 768 || (heavy_pair_ok && cg == 2))) ||
+                     (epi == 2 && cg == 1 && p.k_iters <= 4);
   return launch_gemm(p, BN, 64, a_mn_major != 0, b_mn_major != 0, (cudaStream_t)stream, epi, cg, false, use16 ? 16 : 8);
 }
 
@@ -479,47 +508,24 @@ extern "C" int passl_b200_gemm_stats_rows(void) { return 4 * num_sms(); }
 // ==============================================================================================
 static int conv_fwd_impl(const void* x, const void* w, void* out, int N, int H, int W, int Cin, int Cout, int R, int S,
                          int stride, int pad_h, int pad_w, int Ho, int Wo, const float* bias, const void* residual, int act,
-                         float* col_sum, float* col_sqsum, void* stream) {
+                         float* col_sum, void* stream) {
   if (Cin % 64 || Cout % 8 || R * S > kMaxTaps) return PB_ERR_UNSUPPORTED;
-  const int pad = pad_h;
-  GemmParams p;
-  memset(&p, 0, sizeof(p));
   if (R == 1 && S == 1 && stride == 1 && pad_h == 0 && pad_w == 0 && Ho == H && Wo == W) {
     return passl_b200_gemm_bf16(x, w, out, N * H * W, Cout, Cin, 0, 0, Cin, Cin, Cout, 0, 0, bias, residual, act,
-                                1.f, 1, col_sum, col_sqsum, stream);
+                                1.f, 1, col_sum, nullptr, stream);
   }
+  GemmParams p;
+  memset(&p, 0, sizeof(p));
   for (int r = 0; r < R; ++r)
     for (int s = 0; s < S; ++s) {
       int t = r * S + s;
-      int th = r - pad, tw = s - pad_w;
+      int th = r - pad_h, tw = s - pad_w;
       p.a.dh[t] = (signed char)floordiv(th, stride);
       p.a.dw[t] = (signed char)floordiv(tw, stride);
       p.a.map[t] = (signed char)(stride == 1 ? 0 : posmod(th, 2) * 2 + posmod(tw, 2));
     }
-  const bool halo = stride == 1 && Ho == H && Wo == W && !residual && conv_halo_ok(H, W, R * S, p.a.dh, p.a.dw, p.halo_dh0, p.halo_dw0);
-  if (halo) halo_geom(p.geom, N, Ho, Wo);
-  else pick_patch(p.geom, N, Ho, Wo);
-  p.M = N * Ho * Wo; p.N = Cout;
-  p.m_blocks = p.geom.nb * p.geom.hb * p.geom.wb;
-  int BN = pick_bn(p.m_blocks, Cout);
-  p.n_blocks = (Cout + BN - 1) / BN;
-  p.splits = 1;
-  p.a.mode = OP_PATCH_K;
-  p.a.cchunks = Cin / 64;
-  p.a.ntaps = R * S;
-  p.a.tx_bytes = p.geom.TN * p.geom.TH * p.geom.TW * 128;
-  int rc = halo ? fill_halo_map(p.a, x, N, H, W, Cin) : fill_patch_maps(p.a, x, N, H, W, Cin, stride, p.geom);
-  if (rc) return rc;
-  p.k_iters = R * S * p.a.cchunks;
-  p.k_steps = 4;
-  // (CTA pairs on the 64-wide halo tiles were measured and dropped: 64 ch at 56x56 forward 453 -> 545 us, dgrad 427 -> 501 us)
-  const int cg = pair_eligible(p, BN, 64, false) ? 2 : 1;
-  rc = fill_mat_operand(p.b, w, false, Cout, (long long)R * S * Cin, (long long)R * S * Cin, BN / cg, 64);
-  if (rc) return rc;
-  set_epilogue(p, out, Cout, 0, 0, bias, residual, act, 1.f, col_sum, col_sqsum);
-  p.out_pixel = 1; p.OH = Ho; p.OW = Wo; p.osh = 1; p.osw = 1; p.oh0 = 0; p.ow0 = 0;
-  const int hepi = halo ? halo_lean_epi(p, BN, cg, out, N, Ho, Wo, Cout, residual, act, col_sum) : 0;
-  return launch_gemm(p, BN, 64, false, false, (cudaStream_t)stream, hepi, cg, halo);
+  return conv_igemm(p, x, N, H, W, Cin, stride, R * S, w, Cout, out, Ho, Wo, 1, 0, 0, bias, residual, act, col_sum, false,
+                    (cudaStream_t)stream);
 }
 
 extern "C" int passl_b200_conv2d_fwd_bf16(const void* x, const void* w, void* out, int N, int H, int W, int Cin,
@@ -527,8 +533,7 @@ extern "C" int passl_b200_conv2d_fwd_bf16(const void* x, const void* w, void* ou
                                           const void* residual, int act, float* col_sum, float* col_sqsum,
                                           void* stream) {
   const int Ho = (H + 2 * pad - R) / stride + 1, Wo = (W + 2 * pad - S) / stride + 1;
-  return conv_fwd_impl(x, w, out, N, H, W, Cin, Cout, R, S, stride, pad, pad, Ho, Wo, bias, residual, act, col_sum, col_sqsum,
-                       stream);
+  return conv_fwd_impl(x, w, out, N, H, W, Cin, Cout, R, S, stride, pad, pad, Ho, Wo, bias, residual, act, col_sum, stream);
 }
 
 // Rectangular filters with separate row / column padding and an explicit output extent (stride 1): the W-unfolded
@@ -537,7 +542,7 @@ extern "C" int passl_b200_conv2d_fwd_rect_bf16(const void* x, const void* w, voi
                                                int Cout, int R, int S, int pad_h, int pad_w, int Ho, int Wo,
                                                const float* bias, int act, float* col_sum, void* stream) {
   if (Ho <= 0 || Wo <= 0 || Ho > H + 2 * pad_h - R + 1 + R || Wo > W + 2 * pad_w - S + 1 + S) return PB_ERR_BAD_ARG;
-  return conv_fwd_impl(x, w, out, N, H, W, Cin, Cout, R, S, 1, pad_h, pad_w, Ho, Wo, bias, nullptr, act, col_sum, nullptr, stream);
+  return conv_fwd_impl(x, w, out, N, H, W, Cin, Cout, R, S, 1, pad_h, pad_w, Ho, Wo, bias, nullptr, act, col_sum, stream);
 }
 
 // ==============================================================================================
@@ -628,31 +633,9 @@ extern "C" int passl_b200_conv2d_dgrad_bf16(const void* dy, const void* w, void*
     PB_LAUNCH_CHECK();
     GemmParams p;
     memset(&p, 0, sizeof(p));
-    const int Hc = H / stride, Wc = W / stride;  // class pixel grid
-    for (int t = 0; t < k.ntaps; ++t) { p.a.dh[t] = (signed char)k.dh[t]; p.a.dw[t] = (signed char)k.dw[t]; p.a.map[t] = 0; }
-    const bool halo = stride == 1 && Ho == H && Wo == W && conv_halo_ok(Ho, Wo, k.ntaps, p.a.dh, p.a.dw, p.halo_dh0, p.halo_dw0);
-    if (halo) halo_geom(p.geom, N, Hc, Wc);
-    else pick_patch(p.geom, N, Hc, Wc);
-    p.M = N * Hc * Wc; p.N = Cin;
-    p.m_blocks = p.geom.nb * p.geom.hb * p.geom.wb;
-    int BN = pick_bn(p.m_blocks, Cin);
-    p.n_blocks = (Cin + BN - 1) / BN;
-    p.splits = 1;
-    p.a.mode = OP_PATCH_K;
-    p.a.cchunks = Cout / 64;
-    p.a.ntaps = k.ntaps;
-    p.a.tx_bytes = p.geom.TN * p.geom.TH * p.geom.TW * 128;
-    int rc = halo ? fill_halo_map(p.a, dy, N, Ho, Wo, Cout) : fill_patch_maps(p.a, dy, N, Ho, Wo, Cout, 1, p.geom);
-    if (rc) return rc;
-    p.k_iters = k.ntaps * p.a.cchunks;
-    p.k_steps = 4;
-    const int cg = pair_eligible(p, BN, 64, false) ? 2 : 1;
-    rc = fill_mat_operand(p.b, wt, false, Cin, (long long)k.ntaps * Cout, (long long)k.ntaps * Cout, BN / cg, 64);
-    if (rc) return rc;
-    set_epilogue(p, dx, Cin, 0, 0, nullptr, accumulate ? dx : nullptr, ACT_NONE, 1.f, nullptr, nullptr);
-    p.out_pixel = 1; p.OH = H; p.OW = W; p.osh = stride; p.osw = stride; p.oh0 = k.a; p.ow0 = k.b;
-    const int hepi = halo ? halo_lean_epi(p, BN, cg, dx, N, H, W, Cin, accumulate ? dx : nullptr, ACT_NONE, nullptr) : 0;
-    rc = launch_gemm(p, BN, 64, false, false, st, hepi, cg, halo);
+    for (int t = 0; t < k.ntaps; ++t) { p.a.dh[t] = (signed char)k.dh[t]; p.a.dw[t] = (signed char)k.dw[t]; }
+    const int rc = conv_igemm(p, dy, N, Ho, Wo, Cout, 1, k.ntaps, wt, Cin, dx, H, W, stride, k.a, k.b, nullptr,
+                              accumulate ? dx : nullptr, ACT_NONE, nullptr, true, st);
     if (rc) return rc;
     wt += (size_t)Cin * k.ntaps * Cout;
   }
@@ -724,7 +707,7 @@ static int conv_wgrad_impl(const void* x, const void* dy, float* dw, int N, int 
     }
   rc = fill_patch_maps(p.b, x, N, H, W, Cin, stride, p.geom);
   if (rc) return rc;
-  set_epilogue(p, dw, (long long)R * S * Cin, 1, 1, nullptr, nullptr, ACT_NONE, 1.f, nullptr, nullptr);
+  set_epilogue(p, dw, (long long)R * S * Cin, 1, 1, nullptr, nullptr, ACT_NONE, 1.f, nullptr);
   return launch_gemm(p, BN, 128, true, true, st);
 }
 

@@ -32,7 +32,6 @@
 #include "host_utils.h"
 #include "../../include/passl_b200.h"
 
-#include <stdlib.h>
 #include <string.h>
 
 namespace pb {
@@ -43,6 +42,9 @@ constexpr float kLn2 = 0.6931471805599453f;
 constexpr float kRefShift = 64.f;   // slice sums are accumulated relative to 2^(target + 64): no underflow, overflow only if a
                                     // logit exceeds the target by > 130 nats (then clamped: loss finite, > 100)
 constexpr float kMagic = 12582912.f;  // 1.5 * 2^23
+// exponent mix of the unmasked tiles: one exponential in kPolyEvery on the FMA-pipe polynomial, the others on MUFU (C3 shape,
+// us per forward: MUFU only 15.70, 1/4 15.02, 1/3 15.24, 3/8 15.25)
+constexpr int kPolyEvery = 4;
 
 struct InfoNceTcParams {
   CUtensorMap q_map;  // [N, D] bf16, box {64, 128}
@@ -359,7 +361,7 @@ __device__ __forceinline__ void nce_setup(const InfoNceTcParams& p, const NceSme
 // =====================================================================================================================
 // forward
 // =====================================================================================================================
-template <int MB, int PN, int PD>
+template <int MB>
 __global__ void __launch_bounds__(64 + 128 * MB, 1) infonce_tc_fwd_kernel(const __grid_constant__ InfoNceTcParams p) {
   extern __shared__ uint8_t smem_raw[];
   __shared__ float red[3][4 * MB + 2];
@@ -502,13 +504,13 @@ __global__ void __launch_bounds__(64 + 128 * MB, 1) infonce_tc_fwd_kernel(const 
         if (mn > m) { l *= ex2_mufu(m - mn); m = mn; }
         const float negm = -mn, C = kMagic - mn;
         float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;
-        if (PN > 0 && p.poly_ok) {
+        if (p.poly_ok) {
 #pragma unroll
           for (int j = 0; j < 64; j += 4) {
 #pragma unroll
             for (int u = 0; u < 4; ++u) {
               const float a = __uint_as_float(v[j + u]);
-              const float e = (((j + u) % PD) < PN) ? ex2_poly(a, c2, C) : ex2_mufu(fmaf(a, c2, negm));
+              const float e = ((j + u) % kPolyEvery == 0) ? ex2_poly(a, c2, C) : ex2_mufu(fmaf(a, c2, negm));
               if (u == 0) s0 += e; else if (u == 1) s1 += e; else if (u == 2) s2 += e; else s3 += e;
             }
           }
@@ -611,7 +613,7 @@ __global__ void __launch_bounds__(64 + 128 * MB, 1) infonce_tc_fwd_kernel(const 
 //   dQ_i = scale * g * ( sum_j p_ij K_j  +  (p_i,pos - 1) k+_i   |   - K[label_i] ),   p_ij = exp(scale <q_i,K_j> - lse_i),
 //   g = dloss * loss_scale / N.   P tiles are rounded to bf16 for the second MMA (fp32 accumulation in TMEM).
 // =====================================================================================================================
-template <int MB, int PN, int PD>
+template <int MB>
 __global__ void __launch_bounds__(64 + 128 * MB, 1) infonce_tc_bwd_kernel(const __grid_constant__ InfoNceTcParams p) {
   extern __shared__ uint8_t smem_raw[];
   const NceSmem s = nce_carve(smem_raw, MB, p.D);
@@ -727,12 +729,12 @@ __global__ void __launch_bounds__(64 + 128 * MB, 1) infonce_tc_bwd_kernel(const 
       const bool special = (key0 + NCE_BK > p.K) || (ex >= key0 && ex < key0 + NCE_BK);
       uint32_t w[32];
       if (!__any_sync(0xffffffffu, special)) {
-        if (PN > 0 && p.poly_ok) {
+        if (p.poly_ok) {
 #pragma unroll
           for (int j = 0; j < 64; j += 2) {
             const float a0 = __uint_as_float(v[j]), a1 = __uint_as_float(v[j + 1]);
-            const float e0 = ((j % PD) < PN) ? ex2_poly(a0, c2, C) : ex2_mufu(fmaf(a0, c2, negL));
-            const float e1 = (((j + 1) % PD) < PN) ? ex2_poly(a1, c2, C) : ex2_mufu(fmaf(a1, c2, negL));
+            const float e0 = (j % kPolyEvery == 0) ? ex2_poly(a0, c2, C) : ex2_mufu(fmaf(a0, c2, negL));
+            const float e1 = ((j + 1) % kPolyEvery == 0) ? ex2_poly(a1, c2, C) : ex2_mufu(fmaf(a1, c2, negL));
             w[j >> 1] = pack_bf16x2(e0, e1);
           }
         } else {
@@ -826,17 +828,6 @@ static void nce_plan(int N, int K, int D, int& MB, int& groups, int& slices, int
   smem = q_bytes + stages * stage_bytes + 512 + 1024 + 1024;   // rings + barrier block + target staging + alignment slack
 }
 
-// exponent mix: index into {MUFU only, 1/4, 1/3, 3/8 of the exponentials on the FMA pipe}; PASSL_B200_NCE_POLY overrides
-static int nce_poly_variant() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("PASSL_B200_NCE_POLY");
-    v = e ? atoi(e) : 1;            // measured (C3 shape, us per forward): 15.70 / 15.02 / 15.24 / 15.25 for 0 / 1 / 2 / 3
-    if (v < 0 || v > 3) v = 1;
-  }
-  return v;
-}
-
 template <typename KernelT>
 static int nce_launch(KernelT kern, const InfoNceTcParams& p, int grid, int threads, int smem, cudaStream_t st) {
   PB_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));   // + static smem <= 227 KB
@@ -927,15 +918,8 @@ static int nce_fwd_impl(const void* Q, const void* Kmat, const float* P, const l
   p.lse = lse; p.tgt = tgt; p.loss_rows = loss_rows; p.out = out_scalars;
   p.dbg = g_nce_dbg;
   const int grid = p.row_groups * p.slices, threads = 64 + 128 * MB;
-  const int pv = nce_poly_variant();
-#define NCE_FWD_CASE(mb, pn, pd) rc = nce_launch(infonce_tc_fwd_kernel<mb, pn, pd>, p, grid, threads, smem, st)
-  if (MB == 2) {
-    if (pv == 0) NCE_FWD_CASE(2, 0, 1); else if (pv == 1) NCE_FWD_CASE(2, 1, 4); else if (pv == 2) NCE_FWD_CASE(2, 1, 3); else NCE_FWD_CASE(2, 3, 8);
-  } else {
-    if (pv == 0) NCE_FWD_CASE(1, 0, 1); else if (pv == 1) NCE_FWD_CASE(1, 1, 4); else if (pv == 2) NCE_FWD_CASE(1, 1, 3); else NCE_FWD_CASE(1, 3, 8);
-  }
-#undef NCE_FWD_CASE
-  return rc;
+  return MB == 2 ? nce_launch(infonce_tc_fwd_kernel<2>, p, grid, threads, smem, st)
+                 : nce_launch(infonce_tc_fwd_kernel<1>, p, grid, threads, smem, st);
 }
 
 extern "C" int passl_b200_infonce_tc_fwd(const void* Q, const void* Kmat, const float* P, const long long* label,
@@ -979,12 +963,8 @@ static int nce_bwd_impl(const void* Q, const void* Kmat, const float* P, const l
   p.lse_in = lse; p.tgt_in = tgt; p.dloss = dloss; p.dq = dQ;
   PB_CUDA_CHECK(cudaMemsetAsync(dQ, 0, (size_t)N * D * 4, st));
   const int grid = p.row_groups * p.slices, threads = 64 + 128 * MB;
-  const int pv = nce_poly_variant();
-  if (MB == 2) rc = pv == 0 ? nce_launch(infonce_tc_bwd_kernel<2, 0, 1>, p, grid, threads, smem, st)
-                            : nce_launch(infonce_tc_bwd_kernel<2, 1, 4>, p, grid, threads, smem, st);
-  else rc = pv == 0 ? nce_launch(infonce_tc_bwd_kernel<1, 0, 1>, p, grid, threads, smem, st)
-                    : nce_launch(infonce_tc_bwd_kernel<1, 1, 4>, p, grid, threads, smem, st);
-  return rc;
+  return MB == 2 ? nce_launch(infonce_tc_bwd_kernel<2>, p, grid, threads, smem, st)
+                 : nce_launch(infonce_tc_bwd_kernel<1>, p, grid, threads, smem, st);
 }
 
 extern "C" int passl_b200_infonce_tc_bwd(const void* Q, const void* Kmat, const float* P, const long long* label,

@@ -18,6 +18,8 @@
 
 #include <string.h>
 
+#include <functional>
+
 namespace pb {
 
 constexpr int WH_TH = 8, WH_TW = 16;                        // pixel tile (one image)
@@ -210,10 +212,8 @@ __global__ void __launch_bounds__(192, 1) wgrad_halo_kernel(const __grid_constan
   }
 }
 
-int splitk_scratch(float** out, size_t n_floats, cudaStream_t st);     // gemm_api.cu
-int splitk_release(float* ptr, cudaStream_t st);
-int splitk_reduce(float* out, const float* part, long long rows, long long cols, long long ld, long long stride, int splits,
-                  cudaStream_t st);
+int splitk_run(float* out, long long rows, long long cols, long long ld, int splits, cudaStream_t st,   // gemm_api.cu
+               const std::function<int(float*)>& launch);
 
 int g_wgrad_halo_mode = 0;   // 0 auto (size heuristic), 1 always when the shape is supported, 2 never
 
@@ -225,9 +225,7 @@ int launch_wgrad_halo(const void* x, const void* dy, float* dw, int N, int H, in
   memset(&p, 0, sizeof(p));
   p.dw = dw; p.N = N; p.H = H; p.W = W; p.Cin = Cin; p.Cout = Cout;
   p.R = R; p.S = S; p.pad_h = pad_h; p.pad_w = pad_w;
-  static int cib_env = -1;
-  if (cib_env < 0) { const char* e = getenv("PASSL_B200_WGRAD_HALO_CIB"); cib_env = e ? atoi(e) : 0; }
-  p.cib = (Cin % 128 == 0 && cib_env != 1) ? 2 : 1;
+  p.cib = Cin % 128 == 0 ? 2 : 1;
   const int tmax = p.cib == 2 ? 3 : 5;               // taps per group: 512 TMEM columns / (64 * cib)
   p.groups = (R * S + tmax - 1) / tmax;
   p.tpg = (R * S + p.groups - 1) / p.groups;
@@ -269,24 +267,14 @@ int launch_wgrad_halo(const void* x, const void* dy, float* dw, int N, int H, in
   }
   const int items = base * splits;
   const int grid = items < num_sms() ? items : num_sms();
-  const long long wsize = (long long)Cout * R * S * Cin;
-  if (splits > 1) {
-    int rc = splitk_scratch(&p.partial, (size_t)splits * wsize, st);
-    if (rc) return rc;
-  }
-  wgrad_halo_kernel<<<grid, 192, WH_SMEM, st>>>(p);
-  passl_b200_launch_counter_add(1);
-  const cudaError_t launched = cudaGetLastError();
-  if (launched != cudaSuccess) {
-    if (p.partial) splitk_release(p.partial, st);
-    return (int)launched;
-  }
-  if (splits > 1) {
-    int rc = splitk_reduce(dw, p.partial, Cout, R * S * Cin, R * S * Cin, wsize, splits, st);
-    int rc2 = splitk_release(p.partial, st);
-    return rc ? rc : rc2;
-  }
-  return PB_OK;
+  auto launch = [&](float* partial) -> int {
+    p.partial = partial;
+    wgrad_halo_kernel<<<grid, 192, WH_SMEM, st>>>(p);
+    PB_LAUNCH_CHECK();
+    return PB_OK;
+  };
+  if (splits == 1) return launch(nullptr);
+  return splitk_run(dw, Cout, (long long)R * S * Cin, (long long)R * S * Cin, splits, st, launch);
 }
 
 }  // namespace pb

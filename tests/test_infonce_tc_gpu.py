@@ -111,27 +111,19 @@ def test_state_is_left_clean_between_calls_and_shapes():
                 outs[key] = (o.clone(), lse.clone())
 
 
-@pytest.mark.parametrize("poly", ["0", "1", "2", "3"])
-def test_exponent_mix_variants_agree(poly, monkeypatch):
-    """MUFU-only vs 1/4, 1/3, 3/8 of the exponentials on the FMA-pipe polynomial: same lse to 2e-5."""
-    import subprocess, sys, os
-    code = (
-        "import torch, numpy as np\n"
-        "from passl_b200 import kernels as K\n"
-        "torch.manual_seed(3)\n"
-        "q = torch.nn.functional.normalize(torch.randn(256,128,device='cuda'),dim=1).bfloat16()\n"
-        "k = torch.nn.functional.normalize(torch.randn(65536,128,device='cuda'),dim=1).bfloat16()\n"
-        "p = torch.nn.functional.normalize(torch.randn(256,128,device='cuda'),dim=1)\n"
-        "for T in (0.2, 0.07):\n"
-        "    o, lse, tgt, _ = K.infonce_tc_fwd(q, k, pos=p, scale=1/T)\n"
-        "    S = torch.cat([(q.float()*p).sum(1,keepdim=True), q.float() @ k.float().T], 1).double()/T\n"
-        "    ref = torch.logsumexp(S, 1)\n"
-        "    err = (lse.double()-ref).abs().max().item()\n"
-        "    assert err < 2e-5*ref.abs().max().item()+2e-5, (T, err)\n"
-        "print('ok')\n")
-    env = dict(os.environ, PASSL_B200_NCE_POLY=poly, PYTHONPATH=os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-    r = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=300)
-    assert r.returncode == 0 and "ok" in r.stdout, r.stdout + r.stderr
+def test_exponent_mix_matches_fp64_logsumexp():
+    """1 in 4 of the exponentials on the FMA-pipe polynomial, the rest on MUFU: lse within 2e-5 of the fp64 logsumexp."""
+    from passl_b200 import kernels as K
+    torch.manual_seed(3)
+    q = torch.nn.functional.normalize(torch.randn(256, 128, device="cuda"), dim=1).bfloat16()
+    k = torch.nn.functional.normalize(torch.randn(65536, 128, device="cuda"), dim=1).bfloat16()
+    p = torch.nn.functional.normalize(torch.randn(256, 128, device="cuda"), dim=1)
+    for T in (0.2, 0.07):
+        o, lse, tgt, _ = K.infonce_tc_fwd(q, k, pos=p, scale=1 / T)
+        S = torch.cat([(q.float() * p).sum(1, keepdim=True), q.float() @ k.float().T], 1).double() / T
+        ref = torch.logsumexp(S, 1)
+        err = (lse.double() - ref).abs().max().item()
+        assert err < 2e-5 * ref.abs().max().item() + 2e-5, (T, err)
 
 
 def _ref_dq(qb, kb, pos, label, excl, scale, loss_scale, dloss):
